@@ -4,6 +4,7 @@ CPU baseline and end-to-end (host buffers) numbers.  Contract: see the task stat
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm (N>1: launched by torchrun)
     python bench.py --impl reference [--steps K] [--warmup W]      # the reference's CPU algorithm (oracle port)
+    python bench.py ... --dump-outputs DIR                          # also save the last timed step's outputs (.npy)
 
 Workload (BASELINE.json configs[1], "C2"): one synthetic MaiCity-like HDL-64 scan (64 x 2048 rays) of the
 analytic street scene -> reference-style ray samples (3 surface + 3 free per hit) -> 4-level octree (leaf 0.2 m,
@@ -27,6 +28,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as build() left it (which may be read-only)
 
 METRIC = "sdf_train_points_per_sec_fwd_bwd"
 UNIT = "points/s"
@@ -36,6 +38,8 @@ GATHER_BYTES_PER_POINT = L * 8 * F * 4               # SURVEY.md §8(d): the for
 HBM_FALLBACK_GBS = 6650.0
 C2_POINTS_PER_STEP = 776616   # samples of the C2 scan (64 x 2048 rays, seed 42): the per-GPU step size at every N
 PROFILE_JSON = os.path.join(ROOT, "profiles", "r02_kernel_counters.json")   # ncu-derived per-point counters
+DEC_KEYS = ["layers.0.weight", "layers.0.bias", "layers.1.weight", "layers.1.bias", "lout.weight", "lout.bias"]
+DUMP_BYTES = 64_000_000
 
 
 def workload_config(device):
@@ -366,8 +370,7 @@ def parity_block(orc, o, dec, trainer, octree, decoder, batch, sample, sigma):
     def rel(a, b):
         b = b.double()
         return float((a.detach().cpu().double() - b).abs().max() / b.abs().max().clamp_min(1e-30))
-    keys = ["layers.0.weight", "layers.0.bias", "layers.1.weight", "layers.1.bias", "lout.weight", "lout.bias"]
-    got_dec = dict(zip(keys, trainer.dec_grads))        # views of THIS trainer's flat gradient buffer
+    got_dec = dict(zip(DEC_KEYS, trainer.dec_grads))    # views of THIS trainer's flat gradient buffer
     tg = max(rel(g[:-1], w[:-1]) for g, w in zip(trainer.table_grads, res["table_grads"]))
     dg = max(rel(got_dec[k], w) for k, w in res["dec_grads"].items())
     trainer.zero_grad()
@@ -408,7 +411,7 @@ def hbm_leg(args, dev, peak):
     for i in range(3):
         trainer.zero_grad(); trainer.forward_backward(batches[i][0], batches[i][1], None)
     torch.cuda.synchronize(dev)
-    steps = max(5, min(args.steps, 20))
+    steps = args.steps
     step_ms, kern_ms, red_ms = time_steps(trainer, batches, steps, flush_buf, n, dev, all_reduce=False)
     # forward kernel (hash walk + gather + blend + MLP + loss): the gather figure
     od = octree._descriptor(None, None)
@@ -543,6 +546,29 @@ def other_config_records(dev):
     return out
 
 
+def step_outputs(trainer):
+    """What a training step hands its caller, copied to the host: the loss and the gradient of every table level and
+    decoder tensor (this rank's tables when the map is partitioned)."""
+    out = {"loss": trainer.loss}
+    out.update({f"table_grad_{k}": g for k, g in enumerate(trainer.table_grads)})
+    out.update({"decoder_grad_" + k.replace(".", "_"): g for k, g in zip(DEC_KEYS, trainer.dec_grads) if g is not None})
+    return {k: v.detach().float().cpu().numpy() for k, v in out.items()}
+
+
+def dump_outputs(directory, arrays, budget=DUMP_BYTES):
+    """DIR/<name>.npy for every array.  Beyond `budget` bytes in all, every array keeps the same fraction of its rows,
+    a seeded sample that depends only on the shapes: runs with the same arguments stay comparable row for row."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    frac = min(1.0, (budget - 4096 * len(arrays)) / max(total, 1))     # room for the .npy headers
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        if frac < 1.0 and a.ndim > 0:
+            k = max(1, int(a.shape[0] * frac))
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], k, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_ours(args):
     from shine_mapping_b200 import SdfTrainer, _abi, dist as sdist
     rank, world, local = sdist.init_from_env("nccl")
@@ -613,15 +639,20 @@ def run_ours(args):
     # (SdfTrainer.capture_step) and replayed -- the host only enqueues graph launches; an eager pass with events between
     # the phases follows for the kernel / exchange breakdown
     host_t0 = time.perf_counter()
+    outputs = None
     if graphs is not None:
         step_ms = time_graph_steps(graphs, args.steps, flush_buf, dev)
         launches = _abi.LAUNCHES["count"] - launches0
+        if args.dump_outputs and rank == 0:
+            outputs = step_outputs(trainer)
         sdist.barrier(dev)
         eager_ms, kern_ms, red_ms = time_steps(trainer, batches, args.steps, flush_buf, n_global, dev)
     else:
         step_ms, kern_ms, red_ms = time_steps(trainer, batches, args.steps, flush_buf, n_global, dev)
         eager_ms = step_ms
         launches = _abi.LAUNCHES["count"] - launches0
+        if args.dump_outputs and rank == 0:
+            outputs = step_outputs(trainer)
     sdist.barrier(dev)
     if args.cuda_profiler:
         torch.cuda.profiler.stop()
@@ -773,6 +804,8 @@ def run_ours(args):
                                                            "timed oracle steps (Python-dict lookup + torch CPU autograd)"}
         line["parity"] = parity_block(orc, o, dec, trainer, octree, decoder, sub[0], sample, cfg.sigma_sigmoid)
         line["configs"] = other_config_records(dev)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
 
 
@@ -802,15 +835,15 @@ def main():
     ap.add_argument("--hbm-only", action="store_true", help="run only the HBM-bound leg and print its object (ncu target)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cuda-profiler", action="store_true", help="cudaProfilerStart/Stop around the timed steps")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last timed step's loss and gradients as DIR/<name>.npy "
+                         "(float32; a seeded sample of rows beyond 64 MB in all)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)
     else:
-        import contextlib
-        import __graft_entry__ as ge
-        if int(os.environ.get("LOCAL_RANK", "0")) == 0:
-            with contextlib.redirect_stdout(sys.stderr):      # stdout carries exactly one JSON line
-                ge.build()
+        from shine_mapping_b200 import _abi
+        _abi.lib()      # the kernels build() compiled: the benchmark compiles nothing and writes nothing into the tree
         if args.hbm_only:
             dev = torch.device("cuda", 0)
             torch.cuda.set_device(dev)

@@ -167,6 +167,54 @@ def make_eikonal(name, feat_levels, n_azimuth, n_batch, seed, poly=True, weight_
           f"({os.path.getsize(path) / 1e6:.2f} MB)")
 
 
+def make_live(levels, frames, poly, sample_rows=64):
+    """The reference classes on a seeded `tests.parity_utils.make_case` case (the oracle's initial tables and decoder
+    copied in), frozen for tests/test_reference_live.py.  The table gradients are kept small: per level the set of rows
+    with a nonzero gradient (bit-packed), one weighted sum over the features of each of those rows (seeded weights), and
+    a fixed seeded sample of whole rows plus the trash row."""
+    SHINEConfig, FeatureOctree, Decoder, _, sdf_bce_loss = import_reference()
+    sys.path.insert(0, ROOT)
+    from tests.parity_utils import live_golden_name, make_case
+    case = make_case(n_points=1200, n_batch=1000, feat_levels=levels, seed=77 + levels, n_frames=frames, poly=poly)
+    c = SHINEConfig(); c.device = "cpu"
+    c.tree_level_world, c.tree_level_feat, c.leaf_vox_size, c.poly_int_on = 12, levels, 0.2, poly
+    c.calculate_world_scale()
+    octree, dec = FeatureOctree(c), Decoder(c)
+    for fr in case["frames"]:
+        octree.update(torch.from_numpy(fr), False)
+    assert [tuple(p.shape) for p in octree.hier_features] == [t.shape for t in case["tables"]]
+    with torch.no_grad():
+        for p, t in zip(octree.hier_features, case["tables"]):
+            p.copy_(torch.from_numpy(t))
+    sd = dec.state_dict()
+    for k, v in case["dec"].items():
+        sd[k] = torch.from_numpy(v)
+    dec.load_state_dict(sd)
+    coord, label = torch.from_numpy(case["coord"]), torch.from_numpy(case["label"])
+    pred = dec.sdf(octree.query_feature(coord))
+    loss = sdf_bce_loss(pred, label, case["cfg"]["sigma"], None, False, "mean")
+    loss.backward()
+    out = {"table_rows": np.array([p.shape[0] for p in octree.hier_features]),
+           "exp_pred": pred.detach().numpy(), "exp_loss": np.array(float(loss.detach()))}
+    rng = np.random.default_rng(0)
+    out["tgrad_row_weights"] = w = rng.uniform(0.5, 1.5, case["cfg"]["feature_dim"])
+    for k, p in enumerate(octree.hier_features):
+        g = p.grad.numpy()
+        touched = np.abs(g).sum(1) > 0
+        nz = np.flatnonzero(touched)
+        rows = np.union1d(rng.choice(nz, min(nz.size, sample_rows), replace=False), [g.shape[0] - 1])
+        out[f"exp_tgrad_touched_{k}"] = np.packbits(touched)
+        out[f"exp_tgrad_rows_{k}"] = rows.astype(np.int32)
+        out[f"exp_tgrad_{k}"] = g[rows]
+        out[f"exp_tgrad_rowsum_{k}"] = (g[nz].astype(np.float64) @ w).astype(np.float32)
+    for i, idx in enumerate(octree.hierarchical_indices):
+        assert int(idx.max()) < 2 ** 15
+        out[f"exp_indices_{i}"] = idx.numpy().astype(np.int16)
+    path = os.path.join(ROOT, "tests", "golden", live_golden_name(levels, frames, poly) + ".npz")
+    np.savez_compressed(path, **out)
+    print(f"{path}: N={coord.shape[0]} loss={float(loss.detach()):.6f} ({os.path.getsize(path) / 1e6:.3f} MB)")
+
+
 if __name__ == "__main__":
     if not os.path.isdir(REF):
         sys.exit(f"{REF} not found: goldens can only be minted where the reference is mounted")
@@ -176,3 +224,5 @@ if __name__ == "__main__":
     make("ref_incre_l3_sum_weighted_linear", feat_levels=3, n_frames=2, n_azimuth=10, n_batch=1200, seed=44,
          poly=False, weighted=True, reduction="sum")
     make_eikonal("ref_eikonal_l3", feat_levels=3, n_azimuth=10, n_batch=1000, seed=45)
+    for levels, frames, poly in [(2, 1, True), (4, 2, True), (3, 2, False)]:
+        make_live(levels, frames, poly)

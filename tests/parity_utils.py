@@ -226,6 +226,11 @@ GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
 GOLDEN_NAMES = ["ref_c1_l2_mean", "ref_c2_l4_pretrained_frozen", "ref_incre_l3_sum_weighted_linear"]
 
 
+def live_golden_name(levels, frames, poly):
+    """Golden of the reference classes run on a `make_case` case (oracle/make_golden.py::make_live)."""
+    return f"ref_live_l{levels}_f{frames}_{'poly' if poly else 'linear'}"
+
+
 def load_golden(name):
     """-> (case, expected) frozen from the unmodified reference by oracle/make_golden.py."""
     import json
